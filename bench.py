@@ -2,7 +2,7 @@
 """
 bench.py -- raw-signal samples/sec basecalled (forward + decode) on synthetic chunks.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload all|hac|sup]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload all|hac|sup] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline workload (BASELINE.json configs[1], the one the metric is quoted on): hac-shaped LSTM-CRF (H=384, 5-mer scores,
@@ -43,6 +43,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 
 METRIC = "raw-signal samples/sec basecalled (forward+decode), 10k-sample chunks, hac-shaped LSTM-CRF"
 CHUNK = 10000
@@ -185,6 +186,7 @@ def time_resident(ctx, step, steps, warmup, sampler=None, slots=1):
     W untimed + exactly K timed steps, CUDA events on the launch stream, barrier + synchronize on both sides.
     slots > 1: step i is enqueued on stream i % slots with buffer set i % slots (what score_batches does): consecutive
     batches overlap on the device; the timed region still contains exactly K complete steps.
+    Returns (elapsed ms, events, host enqueue ms per step, what the last timed step returned).
     """
     main = torch.cuda.current_stream()
     from bonito_b200 import native
@@ -208,8 +210,9 @@ def time_resident(ctx, step, steps, warmup, sampler=None, slots=1):
     for st in streams:
         st.wait_event(t0)
     h0 = time.perf_counter()
-    for i in range(steps):
+    for i in range(steps - 1):
         run(i, events)
+    last = run(steps - 1, events)     # only the last step's outputs are kept (the others are released as they are made)
     enqueue_ms = (time.perf_counter() - h0) * 1e3 / steps
     for st in streams:
         main.wait_stream(st)
@@ -217,7 +220,7 @@ def time_resident(ctx, step, steps, warmup, sampler=None, slots=1):
     ctx.barrier()
     if sampler is not None:
         sampler.mark_end()
-    return t0.elapsed_time(t1), events, enqueue_ms
+    return t0.elapsed_time(t1), events, enqueue_ms, last
 
 
 def time_e2e(ctx, model, host_batch, steps, qs):
@@ -236,6 +239,33 @@ def time_e2e(ctx, model, host_batch, steps, qs):
     assert n_out == host_batch.shape[0] * steps
     ctx.barrier()
     return ms
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(directory, scores, decoded):
+    """
+    `--dump-outputs DIR`: what the timed step computed in its last step, as float32 .npy files, so that two builds can be
+    compared output for output (the inputs and weights are seeded, so the same arguments give the same inputs):
+      moves.npy, sequence.npy, qstring.npy  [N, T] the decoder's outputs (what score_batches hands to basecall())
+      scores.npy                            [S, T, C] the scores of S chunks, a fixed seeded sample of the N chunks, as many
+                                            as fit in DUMP_BYTES with the rest
+      scores_chunks.npy                     [S] which chunks those are
+    """
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    arrays = {name: t.cpu().numpy().astype(np.float32) for name, t in zip(("moves", "sequence", "qstring"), decoded)}
+    n, t, c = scores.shape
+    room = DUMP_BYTES - sum(a.nbytes for a in arrays.values()) - 4 * n - 5 * 4096     # chunk list, .npy headers
+    if room < t * c * 4:
+        raise SystemExit(f"--dump-outputs: batch {n} leaves no room for the scores of one chunk in {DUMP_BYTES} bytes")
+    rows = np.sort(np.random.default_rng(0).choice(n, min(n, room // (t * c * 4)), replace=False))
+    arrays["scores"] = scores[torch.from_numpy(rows).to(scores.device)].float().cpu().numpy()
+    arrays["scores_chunks"] = rows.astype(np.float32)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+    log(f"outputs of the last timed step -> {directory}: " + ", ".join(f"{k} {list(a.shape)}" for k, a in arrays.items()))
 
 
 def stage_table(events, steps):
@@ -265,12 +295,15 @@ def bench_hac(ctx, peaks, sampler):
 
     def step(events, slot):
         scores = plan.forward(x_dev, events=events, slot=slot)
-        return _decoder(scores, spec["state_len"], blank_score=plan.blank_score, qscale=qs["scale"], qbias=qs["bias"],
-                        events=events, slot=slot)
+        return scores, _decoder(scores, spec["state_len"], blank_score=plan.blank_score, qscale=qs["scale"],
+                                qbias=qs["bias"], events=events, slot=slot)
 
     slots = N_SLOTS if plan.supports_slots else 1
-    elapsed_ms, events, enqueue_ms = time_resident(ctx, step, args.steps, max(args.warmup, 3), sampler, slots=slots)
+    elapsed_ms, events, enqueue_ms, last = time_resident(ctx, step, args.steps, max(args.warmup, 3), sampler, slots=slots)
     log(f"hac resident: {elapsed_ms / args.steps:.2f} ms/step ({slots} batches in flight)")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
+    del last
     e2e_ms = time_e2e(ctx, model, host_batch, args.steps, qs)
     for _ in range(2):
         compute_scores(model, host_batch, scale=qs["scale"], offset=qs["bias"])
@@ -366,7 +399,7 @@ def bench_hac_quantized(ctx):
         return _decoder(scores, spec["state_len"], blank_score=plan.blank_score, qscale=qs["scale"], qbias=qs["bias"], slot=slot)
 
     steps = min(args.steps, 10)
-    elapsed_ms, _, _ = time_resident(ctx, step, steps, 3, None, slots=N_SLOTS if plan.supports_slots else 1)
+    elapsed_ms, _, _, _ = time_resident(ctx, step, steps, 3, None, slots=N_SLOTS if plan.supports_slots else 1)
     (elapsed_ms,) = ctx.max_over_ranks([elapsed_ms])
     del model, plan
     torch.cuda.empty_cache()
@@ -390,8 +423,9 @@ def sup_flops(spec, plan, N, L):
             "crf_gemm": 2.0 * 2 * M * plan.n_scores * d}, Tq
 
 
-def bench_sup(ctx, peaks, model, spec, L, steps, warmup, with_e2e=True):
-    """One sup configuration: batch 256 x L samples per GPU; returns the block that goes under `configs`."""
+def bench_sup(ctx, peaks, model, spec, L, steps, warmup, with_e2e=True, dump=None):
+    """One sup configuration: batch 256 x L samples per GPU; returns the block that goes under `configs`.
+    `dump`: directory for the outputs of the last timed step (see dump_outputs)."""
     from bonito_b200 import synth
     from bonito_b200.decode import _decoder
     rank, world, device = ctx.rank, ctx.world, ctx.device
@@ -403,12 +437,15 @@ def bench_sup(ctx, peaks, model, spec, L, steps, warmup, with_e2e=True):
 
     def step(events, slot):
         scores = plan.forward(x_dev, events=events, slot=slot)
-        return _decoder(scores, spec["state_len"], blank_score=plan.blank_score, qscale=qs["scale"], qbias=qs["bias"],
-                        events=events, slot=slot)
+        return scores, _decoder(scores, spec["state_len"], blank_score=plan.blank_score, qscale=qs["scale"],
+                                qbias=qs["bias"], events=events, slot=slot)
 
     # one batch at a time: the sup step is one long chain of chip-filling GEMMs, a second batch in flight buys nothing
     # (54.5 vs 56.2 ms measured) and would blur the per-kernel event times
-    elapsed_ms, events, enqueue_ms = time_resident(ctx, step, steps, warmup, slots=1)
+    elapsed_ms, events, enqueue_ms, last = time_resident(ctx, step, steps, warmup, slots=1)
+    if dump and rank == 0:
+        dump_outputs(dump, *last)
+    del last
     e2e_ms = time_e2e(ctx, model, host_batch, steps, qs) if with_e2e else 0.0
     elapsed_ms, e2e_ms = ctx.max_over_ranks([elapsed_ms, e2e_ms])
     log(f"sup L={L}: resident {elapsed_ms / steps:.2f} ms/step" + (f", e2e {e2e_ms / steps:.2f}" if with_e2e else ""))
@@ -573,7 +610,14 @@ def main():
                     help="all: hac headline line + the other BASELINE configurations under `configs`; hac: headline only; "
                          "sup: config 3 as the headline of the line")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (float32, at most "
+                         "64 MB: decoder outputs of every chunk, scores of a seeded sample of chunks; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
 
     rank = int(os.environ.get("RANK", 0))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
@@ -621,7 +665,9 @@ def main():
                     sampler.start()
                     time.sleep(0.3)
                     sampler.mark_begin()
-            c3 = bench_sup(ctx, peaks, model, spec, 9996, sup_steps, sup_warm)
+            headline = args.workload == "sup"
+            c3 = bench_sup(ctx, peaks, model, spec, 9996, args.steps if headline else sup_steps, sup_warm,
+                           dump=args.dump_outputs if headline else None)
             if args.workload == "sup" and rank == 0:
                 sampler.mark_end()
                 clocks = sampler.stop()

@@ -6,6 +6,7 @@ The reference itself has no C/C++ sources to compile (SURVEY.md section 0), so `
 import ctypes
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -16,10 +17,19 @@ _lib = None
 
 
 def build(force=False):
-    if force or not os.path.exists(OUT) or os.path.getmtime(OUT) < os.path.getmtime(SRC):
+    """Path of an up-to-date library, compiled if needed: into oracle/_ref/, or into a temporary directory where the tree
+    cannot be written (bench.py may run from a read-only one)."""
+    if not force and os.path.exists(OUT) and os.path.getmtime(OUT) >= os.path.getmtime(SRC):
+        return OUT
+    out = OUT
+    try:
         os.makedirs(os.path.dirname(OUT), exist_ok=True)
-        subprocess.run(["gcc", "-O2", "-fopenmp", "-shared", "-fPIC", "-o", OUT, SRC, "-lm"], check=True)
-    return OUT
+    except OSError:
+        pass
+    if not os.access(os.path.dirname(OUT), os.W_OK):
+        out = os.path.join(tempfile.mkdtemp(prefix="crf_decode_ref_"), os.path.basename(OUT))
+    subprocess.run(["gcc", "-O2", "-fopenmp", "-shared", "-fPIC", "-o", out, SRC, "-lm"], check=True)
+    return out
 
 
 def load():

@@ -11,13 +11,18 @@ Contents
   forward_sup.npz  narrow transformer through the reference's bonito.transformer classes (Triton / CUDA-only pieces
                    replaced by flash-attn's torch reference functions, see oracle/reference_shim.load_transformer)
   forward_hac.npz  the headline shape (H = 384, 5 LSTM, k = 4) through the reference module tree, fp32 CPU: input, scores
-                   without the blank column [N,T,1024], decode_batch strings, digest of the seeded weights
+                   without the blank column [N,T,1024] (sampled), decode_batch strings, digest of the seeded weights
   revcomp.npz      CTC_CRF.reverse_complement of the reference on small random scores, k = 3, 4, 5
   forward_sup_wide.npz  the sup v5 width (d_model 512, 8 heads, ff 2048, k = 5), 6 layers, through the reference's
-                   bonito.transformer classes: input, conv output, layers 0 and 5, scores [N,2T',4096]; weights by digest
+                   bonito.transformer classes: input, conv output, layers 0 and 5, scores [N,2T',4096] (all sampled);
+                   weights by digest
   forward_fast.npz reference module tree (bonito.nn via from_dict, BatchNorm folded by fuse_bn_) forward in
-                   fp32 on CPU: input, every parameter, per-layer features, scores [T,N,C+blanks];
+                   fp32 on CPU: input, every parameter, per-layer features and scores [T,N,C+blanks] (sampled);
                    + decode_batch strings (reference glue over the oracle's posteriors stand-in)
+
+"Sampled" outputs keep a seeded subset of the indices of their last axis (channels or score columns; every chunk and
+every time step stays), listed beside them as `<name>_idx`: each fixture file stays under 1 MB.  Inputs, parameters and
+decoded strings are always stored whole.
 """
 
 import json
@@ -29,6 +34,16 @@ import torch
 from oracle import reference_shim, synth
 
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
+
+
+def sample_last_axis(out, names, fraction, seed=0):
+    """Replace each named output by a seeded subset of its last axis (sorted indices stored as `<name>_idx`)."""
+    rng = np.random.default_rng(seed)
+    for name in names:
+        n = out[name].shape[-1]
+        idx = np.sort(rng.choice(n, max(1, round(n * fraction)), replace=False)).astype(np.int32)
+        out[name] = np.ascontiguousarray(out[name][..., idx])
+        out[name + "_idx"] = idx
 
 
 class _Read:
@@ -118,6 +133,7 @@ def forward_fast(ref):
     for k, v in model.state_dict().items():
         if ".conv." in k:  # only the convolutions change under fuse_bn_
             out["fused." + k] = v.numpy()
+    sample_last_axis(out, ["scores", "feat_1", "feat_2", "feat_4", "feat_5"], 1 / 6)   # the parameters take half the budget
     np.savez_compressed(os.path.join(OUT, "forward_fast.npz"), **out)
     print("forward_fast.npz scores", tuple(scores.shape), "strings", [len(s) for s in strings])
 
@@ -178,6 +194,7 @@ def forward_hac(ref):
     ntc = s4[..., 1:].reshape(t, n, -1).permute(1, 0, 2).contiguous()
     out = {"x": x.numpy().astype(np.float16), "scores_ntc": ntc.numpy(), "strings": np.array(json.dumps(strings)),
            "digest": np.array(weights_digest(weights)), "seed": np.array(31), "stride": np.array(model.stride)}
+    sample_last_axis(out, ["scores_ntc"], 1 / 2)
     np.savez_compressed(os.path.join(OUT, "forward_hac.npz"), **out)
     print("forward_hac.npz scores", tuple(ntc.shape), "strings", [len(s) for s in strings], "max|s|", float(ntc.abs().max()))
 
@@ -223,6 +240,7 @@ def forward_sup_wide(ref):
     out = {"x": x.numpy().astype(np.float16), "scores_ntc": ntc.numpy(), "conv": conv.numpy(),
            "layer0": layers[0].numpy(), "layer5": layers[5].numpy(), "digest": np.array(weights_digest(weights)),
            "seed": np.array(11), "depth": np.array(6), "stride": np.array(model.stride)}
+    sample_last_axis(out, ["scores_ntc", "conv", "layer0", "layer5"], 1 / 5)
     np.savez_compressed(os.path.join(OUT, "forward_sup_wide.npz"), **out)
     print("forward_sup_wide.npz scores", tuple(ntc.shape), "std %.2f max %.1f" % (float(ntc.std()), float(ntc.abs().max())))
 

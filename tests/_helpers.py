@@ -19,6 +19,11 @@ def edit_distance(a, b):
     return int(prev[-1])
 
 
+def at_sample(full, gold, name):
+    """`full` at the indices of its last axis that the fixture stores `name` at (`<name>_idx`, oracle/make_golden.py)."""
+    return np.asarray(full)[..., gold[name + "_idx"]]
+
+
 def identity(a, b):
     """1 - edit distance / length of the longer string."""
     n = max(len(a), len(b), 1)

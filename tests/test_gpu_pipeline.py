@@ -277,8 +277,8 @@ def test_score_batches_equals_compute_scores():
 
 def test_headline_shape_against_the_reference_fixture(golden_dir):
     """hac shape through the native engine vs scores produced by the reference's own module tree (fp32 CPU,
-    tests/golden/forward_hac.npz): fp16 tolerance on the scores, same base sequences."""
-    from _helpers import identity
+    tests/golden/forward_hac.npz, a sample of its score columns): fp16 tolerance on the scores, same base sequences."""
+    from _helpers import at_sample, identity
     from oracle.make_golden import weights_digest
     from bonito_b200.crf.model import Model
     from bonito_b200.decode import beam_search, to_str
@@ -295,8 +295,9 @@ def test_headline_shape_against_the_reference_fixture(golden_dir):
     with torch.inference_mode():
         scores = model(x)
         seq, _, _ = beam_search(scores)
+    assert scores.shape == (2, 200, 1024)
     ref = torch.from_numpy(gold["scores_ntc"])
-    err = (scores.float().cpu() - ref).abs()
+    err = (torch.from_numpy(at_sample(scores.float().cpu(), gold, "scores_ntc")) - ref).abs()
     print("vs reference fixture: max", err.max().item(), "mean", err.mean().item())
     assert err.max().item() <= 2e-2 and err.mean().item() <= 2e-3
     want = json.loads(str(gold["strings"]))
